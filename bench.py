@@ -45,7 +45,12 @@ def parse():
     ap.add_argument("--parity-mode-multi", action="store_true", help="also time the bf16x3 leg when --gpus > 1")
     ap.add_argument("--optimizer", default="torch", choices=["torch", "fused"],
                     help="torch.optim.SGD (the reference's, tool/train.py:140) or semseg_b200.optim.FusedSGD (one launch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0; B200 arm only)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
+    return args
 
 
 def peaks():
@@ -111,6 +116,36 @@ def synth_batch(n, size, classes, seed):
     y = torch.randint(0, classes, (n, size, size), generator=g)
     y[torch.rand((n, size, size), generator=g) < 0.05] = 255
     return x, y
+
+
+DUMP_MAX_ELEMS = 4 * 1024 * 1024      # per array: 16 MB as float32, so a dump of three arrays and scalars stays < 64 MB
+
+
+def dump_sample(t):
+    """`t` itself when it has at most DUMP_MAX_ELEMS elements, else that many of its elements (flattened) at positions
+    drawn from a fixed seed, the same positions for the same size in every run."""
+    import torch
+    if t.numel() <= DUMP_MAX_ELEMS:
+        return t
+    idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(out_dir, outputs, model):
+    """Writes what one training step hands back, as float32 .npy files: the prediction and both losses of
+    model(input, target), the loss it back-propagated, and the parameter gradients and updated parameters (all
+    parameters flattened in model.parameters() order and sampled by dump_sample)."""
+    import numpy as np
+    import torch
+    pred, main_loss, aux_loss, loss = outputs
+    params = list(model.parameters())
+    grads = [p.grad if p.grad is not None else torch.zeros_like(p) for p in params]
+    arrays = {"pred": dump_sample(pred), "main_loss": main_loss, "aux_loss": aux_loss, "loss": loss,
+              "grads": dump_sample(torch.cat([g.reshape(-1) for g in grads])),
+              "params": dump_sample(torch.cat([p.detach().reshape(-1) for p in params]))}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def build_optimizer(model, arch, kind="torch"):
@@ -285,12 +320,16 @@ def run_b200_arm(args):
     x_dev, y_dev = x_host.to(dev), y_host.to(dev)
     h2d = x_host.numel() * 4 + y_host.numel() * 8
 
+    last = []               # outputs of the latest step, kept for --dump-outputs only
+
     def step(inp, tgt):
-        _, main_loss, aux_loss = model(inp, tgt)
+        pred, main_loss, aux_loss = model(inp, tgt)
         loss = main_loss + 0.4 * aux_loss
         opt.zero_grad()
         loss.backward()
         opt.step()
+        if args.dump_outputs:
+            last[:] = (pred, main_loss, aux_loss, loss)
         return loss
 
     def step_e2e():
@@ -327,6 +366,9 @@ def run_b200_arm(args):
     l0 = _lib.launch_count()
     ms_dev = timed(lambda: step(x_dev, y_dev), args.steps)
     launches = _lib.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        # before any further step: a replayed step graph rewrites the same static output buffers every time
+        dump_outputs(args.dump_outputs, last, inner)
     graphed = graphs.launches_per_step(inner)
     if graphed:                      # kernels replayed from the captured step graphs are not counted by the library
         launches += graphed * args.steps

@@ -57,14 +57,15 @@ def psamask_bwd(dout, psa_type, mask_h, mask_w):
     return din
 
 
-def ref_psamask_module():
-    """The reference's own CPU extension (oracle/_ref/psamask_ref_cpu*.so) or None if it was not built."""
+def ref_psamask_module(device="cpu"):
+    """The reference's own CPU or GPU extension (oracle/_ref/psamask_ref_{cpu,gpu}*.so) or None if it was not built."""
     if not os.path.isdir(_REF_DIR):
         return None
     import torch  # noqa: F401  (the extension links against libtorch)
+    name = "psamask_ref_" + device
     for f in sorted(os.listdir(_REF_DIR)):
-        if f.startswith("psamask_ref_cpu") and f.endswith(".so"):
-            spec = importlib.util.spec_from_file_location("psamask_ref_cpu", os.path.join(_REF_DIR, f))
+        if f.startswith(name) and f.endswith(".so"):
+            spec = importlib.util.spec_from_file_location(name, os.path.join(_REF_DIR, f))
             mod = importlib.util.module_from_spec(spec)
             spec.loader.exec_module(mod)
             return mod

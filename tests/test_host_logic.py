@@ -148,6 +148,30 @@ def test_bench_reference_runner_environment(monkeypatch):
     assert "CUDA_VISIBLE_DEVICES" not in seen["env"] and seen["cmd"][seen["cmd"].index("--threads") + 1] == "8"
 
 
+def test_bench_dump_outputs_writes_float32_and_samples_the_same_positions(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every array is float32; one larger than DUMP_MAX_ELEMS is sampled at the same positions
+    in every run, so that two builds can be compared output for output."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 64)
+    m = torch.nn.Conv2d(3, 8, 3)                      # 224 weights + 8 biases, more than 64
+    for p in m.parameters():
+        p.grad = torch.full_like(p, 0.5)
+    pred = torch.arange(60, dtype=torch.long).reshape(1, 6, 10)
+    outputs = (pred, torch.tensor(1.5), torch.tensor(2.0), torch.tensor(2.3))
+    bench.dump_outputs(str(tmp_path / "a"), outputs, m)
+    bench.dump_outputs(str(tmp_path / "b"), outputs, m)
+    flat = torch.cat([p.detach().reshape(-1) for p in m.parameters()])
+    for name in ("pred", "main_loss", "aux_loss", "loss", "grads", "params"):
+        a, b = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert a.dtype == np.float32 and np.array_equal(a, b), name
+    assert np.array_equal(np.load(tmp_path / "a" / "pred.npy"), pred.float().numpy())
+    assert float(np.load(tmp_path / "a" / "loss.npy")) == np.float32(2.3)
+    grads, params = np.load(tmp_path / "a" / "grads.npy"), np.load(tmp_path / "a" / "params.npy")
+    assert grads.shape == params.shape == (64,) and (grads == 0.5).all()
+    assert np.isin(params, flat.numpy()).all() and len(np.unique(params)) > 32
+
+
 def test_precision_mode_switch_and_graph_gates(monkeypatch):
     """Host-side switches: the operand policy (semseg_b200/precision.py) and the CUDA-graph gate (graphs.enabled /
     train_step declining anything that is not a CUDA training call)."""

@@ -1,11 +1,11 @@
 """CPU tier: pin the oracle (oracle/) against the reference — golden fixtures made from the real reference
-(tests/golden/make_golden.py) and, when built, the reference's own compiled psamask extension (oracle/_ref)."""
+(tests/golden/make_golden.py) and from the reference's own compiled psamask extension
+(tests/golden/make_golden_ext.py)."""
 import hashlib
 import json
 import os
 
 import numpy as np
-import pytest
 import torch
 
 import oracle
@@ -32,21 +32,13 @@ def test_psamask_oracle_matches_reference_goldens(golden_dir):
                 assert np.array_equal(din, g[key + "/din"])
 
 
-def test_psamask_oracle_matches_compiled_reference():
-    ref = oracle.ref_psamask_module()
-    if ref is None:
-        pytest.skip("oracle/_ref not built (reference tree absent)")
-    rng = np.random.default_rng(11)
-    for (n, h, w, mh, mw) in CASES + [(1, 3, 9, 5, 17), (1, 1, 1, 1, 1)]:
-        for t in (0, 1):
-            x = rng.standard_normal((n, mh * mw, h, w)).astype(np.float32)
-            out = torch.zeros(n, h * w, h, w)
-            ref.psamask_forward(t, torch.from_numpy(x), out, n, h, w, mh, mw, (mh - 1) // 2, (mw - 1) // 2)
-            assert np.array_equal(oracle.psamask_fwd(x, t, mh, mw), out.numpy())
-            g = rng.standard_normal((n, h * w, h, w)).astype(np.float32)
-            gi = torch.zeros(n, mh * mw, h, w)
-            ref.psamask_backward(t, torch.from_numpy(g), gi, n, h, w, mh, mw, (mh - 1) // 2, (mw - 1) // 2)
-            assert np.array_equal(oracle.psamask_bwd(g, t, mh, mw), gi.numpy())
+def test_psamask_oracle_matches_compiled_reference(golden_dir):
+    """Bit-identical to the reference's own compiled CPU extension (lib/psa/src/cpu/psamask.cpp), whose outputs
+    tests/golden/make_golden_ext.py recorded in psamask_ref_cpu.npz."""
+    g = np.load(os.path.join(golden_dir, "psamask_ref_cpu.npz"))
+    for key, t, mh, mw, x, dout in util.psamask_cpu_ext_cases():
+        util.check_psamask_golden(g, key, x, dout, oracle.psamask_fwd(x, t, mh, mw),
+                                  oracle.psamask_bwd(dout, t, mh, mw))
 
 
 def test_psamask_torch_restatement_matches_c_oracle():

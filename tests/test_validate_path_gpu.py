@@ -2,6 +2,9 @@
 autograd ENABLED and every parameter requiring grad, followed by `criterion(output, target)`; nothing is back-propagated.
 The eval-mode BatchNorm path folds conv + BN (+ residual, ReLU) into one kernel that has no backward, so it must neither
 raise nor change the numbers relative to the torch.no_grad() call that tool/test.py makes."""
+import os
+
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
@@ -28,37 +31,15 @@ def test_eval_forward_with_autograd_enabled_equals_no_grad(arch):
     assert bool(torch.isfinite(loss))
 
 
-def _load_stock_psamask():
-    """The reference's own CUDA extension (lib/psa/src/gpu/*), compiled in place by oracle/build.py into oracle/_ref/."""
-    import importlib.util
-    import os
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-    for f in sorted(os.listdir(ref_dir)) if os.path.isdir(ref_dir) else []:
-        if f.startswith("psamask_ref_gpu") and f.endswith(".so"):
-            spec = importlib.util.spec_from_file_location("psamask_ref_gpu", os.path.join(ref_dir, f))
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
-            return mod
-    return None
-
-
-@pytest.mark.parametrize("geom", [(2, 30, 30, 59, 59), (1, 9, 12, 9, 7), (3, 5, 40, 9, 79), (1, 13, 13, 25, 25)])
+@pytest.mark.parametrize("geom", util.PSAMASK_EXT_GPU_CASES)
 @pytest.mark.parametrize("psa_type", [0, 1])
-def test_psamask_bit_identical_to_the_references_cuda_kernel(geom, psa_type):
+def test_psamask_bit_identical_to_the_references_cuda_kernel(geom, psa_type, golden_dir):
     """psa_mask forward / backward against the reference's stock GPU kernel (lib/psa/src/gpu/psamask_cuda.cu:8-128) called
-    the way lib/psa/functions/psamask.py:17-35 calls it (zero-filled output, then the kernel): bit-identical."""
+    the way lib/psa/functions/psamask.py:17-35 calls it (zero-filled output, then the kernel): bit-identical. The
+    stock kernel's outputs were recorded on a B200 by tests/golden/make_golden_ext.py (psamask_ref_gpu.npz)."""
     from semseg_b200 import ops
-    stock = _load_stock_psamask()
-    if stock is None:
-        pytest.skip("oracle/_ref/psamask_ref_gpu*.so not built (reference tree or nvcc absent at build time)")
-    n, h, w, mh, mw = geom
-    g = torch.Generator(device="cuda").manual_seed(h * 31 + w + psa_type)
-    x = torch.randn((n, mh * mw, h, w), device="cuda", generator=g)
-    go = torch.randn((n, h * w, h, w), device="cuda", generator=g)
-    out = torch.zeros((n, h * w, h, w), device="cuda")
-    stock.psamask_forward(psa_type, x, out, n, h, w, mh, mw, (mh - 1) // 2, (mw - 1) // 2)
-    gin = torch.zeros((n, mh * mw, h, w), device="cuda")
-    stock.psamask_backward(psa_type, go, gin, n, h, w, mh, mw, (mh - 1) // 2, (mw - 1) // 2)
-    torch.cuda.synchronize()
-    assert torch.equal(ops.psamask_fwd(x, psa_type, mh, mw), out)
-    assert torch.equal(ops.psamask_bwd(go, psa_type, mh, mw), gin)
+    g = np.load(os.path.join(golden_dir, "psamask_ref_gpu.npz"))
+    _, _, _, mh, mw = geom
+    x, go = util.psamask_gpu_ext_inputs(geom, psa_type)
+    util.check_psamask_golden(g, util.psamask_key(geom, psa_type), x, go, ops.psamask_fwd(x, psa_type, mh, mw),
+                              ops.psamask_bwd(go, psa_type, mh, mw))

@@ -1,4 +1,6 @@
 """Shared helpers for the tests (synthetic inputs identical to tests/golden/_ref_worker.py)."""
+import hashlib
+
 import numpy as np
 import torch
 
@@ -77,3 +79,54 @@ def metric_case(seed, shape, K, ignore=255):
 
 
 METRIC_CASES = [(1, (2, 33, 47), 150), (2, (1, 65, 65), 19), (3, (4000,), 2), (4, (3, 17), 300)]
+
+
+# psa_mask geometries (n, h, w, mask_h, mask_w) of the goldens recorded from the reference's own compiled CPU and CUDA
+# extensions (tests/golden/make_golden_ext.py)
+PSAMASK_EXT_CPU_CASES = [(2, 4, 5, 7, 9), (1, 6, 7, 5, 3), (2, 5, 5, 9, 9), (1, 30, 30, 59, 59), (1, 3, 9, 5, 17),
+                         (1, 1, 1, 1, 1)]
+PSAMASK_EXT_GPU_CASES = [(2, 30, 30, 59, 59), (1, 9, 12, 9, 7), (3, 5, 40, 9, 79), (1, 13, 13, 25, 25)]
+
+
+def psamask_key(geom, psa_type):
+    return "n%d_h%d_w%d_mh%d_mw%d_t%d" % (tuple(geom) + (psa_type,))
+
+
+def psamask_cpu_ext_cases():
+    """(key, psa_type, mask_h, mask_w, x, dout) of the CPU-extension goldens (float32 ndarrays, one seeded stream)."""
+    rng = np.random.default_rng(11)
+    for geom in PSAMASK_EXT_CPU_CASES:
+        n, h, w, mh, mw = geom
+        for t in (0, 1):
+            x = rng.standard_normal((n, mh * mw, h, w)).astype(np.float32)
+            dout = rng.standard_normal((n, h * w, h, w)).astype(np.float32)
+            yield psamask_key(geom, t), t, mh, mw, x, dout
+
+
+def psamask_gpu_ext_inputs(geom, psa_type):
+    """(x, dout) of the CUDA-extension goldens, drawn on the GPU from a seeded generator."""
+    n, h, w, mh, mw = geom
+    g = torch.Generator(device="cuda").manual_seed(h * 31 + w + psa_type)
+    x = torch.randn((n, mh * mw, h, w), device="cuda", generator=g)
+    dout = torch.randn((n, h * w, h, w), device="cuda", generator=g)
+    return x, dout
+
+
+def _np(a):
+    return a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(_np(a)).tobytes()).hexdigest()
+
+
+def check_psamask_golden(g, key, x, dout, out, din):
+    """out / din bit-identical to the golden entry `key` (written by tests/golden/make_golden_ext.py), whose inputs must
+    be x / dout."""
+    assert sha256(x) == str(g[key + "/x_sha"]) and sha256(dout) == str(g[key + "/dout_sha"]), \
+        "%s: inputs differ from those the golden was recorded with" % key
+    if key + "/out" in g:
+        assert np.array_equal(_np(out), g[key + "/out"]), key
+        assert np.array_equal(_np(din), g[key + "/din"]), key
+    assert sha256(out) == str(g[key + "/out_sha"]), key
+    assert sha256(din) == str(g[key + "/din_sha"]), key
